@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — masks/sec of the PSALM inference hot path (PSALM.eval_seg) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (BASELINE.json configs[1]): COCO-panoptic prompt with 134 class names, 1024x1024 image,
@@ -32,6 +32,8 @@ single-image latency of the reference's eval scripts, 8.2 ms).
           (`--acc-images` per rank, accumulators all_reduced over ranks; oracle/accuracy.py).
   --impl reference : times that CPU port as the reference arm (the reference is Python and cannot
           travel to the box; its CUDA op has no CPU build — see DESIGN.md).
+  --dump-outputs DIR : after the timed steps of the value arm, writes what its last step returned (rank 0) as
+          DIR/<name>.npy, for an output-by-output comparison of two builds on the same (seeded) inputs.
 """
 import argparse
 import json
@@ -43,7 +45,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the bench leaves the source tree as it found it (it may be read-only)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOAD = "coco-panoptic 1024x1024, 134 class names, 100 queries, Swin-B + Phi-1.5"
@@ -216,19 +220,12 @@ def run_reference(args, rank, world):
     threads = cpu_threads()
     sd = bench_weights(PsalmConfig(), torch.float32)
     inp = bench_inputs(1, 1)
-    times = [oracle_eval(sd, inp, 0, threads, intermediates=False)[0]]       # first image doubles as the cost probe
-    per = times[0]
-    budget = 240.0
-    k_run = max(1, min(K, int((budget - per * (1 + min(W, 1))) / per)))
-    w_run = min(W, 1) if k_run < K else W
-    w_run = min(w_run, max(0, int((budget - per * k_run) / per) - 1))
-    for _ in range(k_run + w_run - 1):
-        times.append(oracle_eval(sd, inp, 0, threads, intermediates=False)[0])
-    timed = times[w_run:] if len(times) > w_run else times
+    times = [oracle_eval(sd, inp, 0, threads, intermediates=False)[0] for _ in range(W + K)]
+    timed = times[W:]
     sec = sum(timed) / len(timed)
     val = 100.0 / sec
     line = {"impl": "reference", "metric": "masks/sec", "value": val, "unit": "masks/s", "n_gpus": args.gpus,
-            "steps": len(timed), "steps_requested": K, "warmup": w_run, "ms_per_step": sec * 1e3,
+            "steps": len(timed), "warmup": W, "ms_per_step": sec * 1e3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": WORKLOAD, "batch_per_gpu": args.batch, "images_per_step": 1,
                        "note": "bounded sample: each step is ONE image of the batch (masks/s is per image); "
@@ -244,6 +241,7 @@ def run_reference(args, rank, world):
 
 # ------------------------------------------------------------------------------------------------
 def timed_device_steps(step, K, W, barrier):
+    """(milliseconds of K timed steps after W warm-up steps, what the last timed step returned)"""
     for _ in range(W):
         step()
     torch.cuda.synchronize()
@@ -252,11 +250,53 @@ def timed_device_steps(step, K, W, barrier):
     torch.cuda.synchronize()
     e0.record()
     for _ in range(K):
-        step()
+        last = step()
     e1.record()
     torch.cuda.synchronize()
     barrier()
-    return e0.elapsed_time(e1)
+    return e0.elapsed_time(e1), last
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(results, image_hw, n_queries, out_dir, seed=0):
+    """Write what one step returned (PSALM.post_process: per image sem_seg [C,H,W], instances, panoptic_seg) to
+    out_dir/<name>.npy.  Every shape depends only on the batch B, the class count C and the query count Q, never on
+    the values, so that two builds run with the same arguments write arrays of the same shapes:
+      pixel_yx [N,2]: a fixed, seeded sample of N pixels, N chosen to keep the files under DUMP_BYTES;
+      panoptic_seg [B,N]: segment id at each sampled pixel;
+      panoptic_segments [B,Q,3]: row k = (id, isthing, category_id) of segment id k + 1, -1 where there is none;
+      sem_seg [B,C,N];
+      instances [B,Q,3]: (score, pred_class, query_index) of each kept instance, then -1 rows;
+      instance_masks [B,Q,N]: the masks of those instances at the sampled pixels, then zero rows."""
+    H, W = image_hw
+    B, C, Q = len(results), results[0]["sem_seg"].shape[0], n_queries
+    n = min(H * W, (DUMP_BYTES - 4 * 10 ** 6) // (4 * B * (1 + C + Q)))
+    pix = torch.from_numpy(np.sort(np.random.default_rng(seed).choice(H * W, n, replace=False)))
+    dev_pix = pix.to(results[0]["sem_seg"].device)
+    segments = np.full((B, Q, 3), -1.0)
+    inst = np.full((B, Q, 3), -1.0)
+    inst_masks = np.zeros((B, Q, n), dtype=np.float32)
+    for b, r in enumerate(results):
+        for s in r["panoptic_seg"][1]:                 # ids are 1 .. number of segments <= Q
+            segments[b, s["id"] - 1] = (s["id"], s["isthing"], s["category_id"])
+        i = r["instances"]
+        k = len(i.scores)                              # <= Q: the top-k of the task heads keeps at most Q
+        inst[b, :k] = torch.stack([i.scores.float(), i.pred_classes.float(), i.query_index.float()], 1).cpu().numpy()
+        inst_masks[b, :k] = i.pred_masks.flatten(1)[:, dev_pix].float().cpu().numpy()
+    arrays = {
+        "pixel_yx": np.stack([pix.numpy() // W, pix.numpy() % W], 1).astype(np.float64),
+        "panoptic_seg": torch.stack([r["panoptic_seg"][0].flatten()[dev_pix] for r in results]).float().cpu().numpy(),
+        "panoptic_segments": segments,
+        "sem_seg": torch.stack([r["sem_seg"].flatten(1)[:, dev_pix] for r in results]).float().cpu().numpy(),
+        "instances": inst,
+        "instance_masks": inst_masks,
+    }
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_ours(args, rank, world, local_rank):
@@ -293,7 +333,10 @@ def run_ours(args, rank, world, local_rank):
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms_total = timed_device_steps(step_device, K, W, barrier)
+    ms_total, last = timed_device_steps(step_device, K, W, barrier)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, (IMG, IMG), model.num_queries, args.dump_outputs)
+    del last
     # outputs of the timed configuration (graph replay at batch B), kept for the parity / accuracy checks below
     out_timed = None
     if not args.no_graph:
@@ -310,7 +353,7 @@ def run_ours(args, rank, world, local_rank):
         def step_b1():
             out = model.forward_core(img1, plan1) if args.no_graph else model.forward_core_graphed(img1, plan1)
             return model.post_process(out, (IMG, IMG), inp["seg_info"][:1])
-        ms1 = PD.max_over_ranks([timed_device_steps(step_b1, K, W, barrier)], dev)[0]
+        ms1 = PD.max_over_ranks([timed_device_steps(step_b1, K, W, barrier)[0]], dev)[0]
         b1 = {"value": K * world * 100.0 / (ms1 / 1e3), "unit": "masks/s", "ms_per_image": ms1 / K, "batch_per_gpu": 1}
 
     # the reference's real eval flow (coco_panoptic_mapper.py:148-162): a 640 x 480 image resized to 1024 x 768, padded to
@@ -325,7 +368,7 @@ def run_ours(args, rank, world, local_rank):
         def step_mapper():
             out = model.forward_core_graphed(images_d, plan_d, fuse_post=fused_m)
             return model.post_process(out, (IMG, IMG), seg_m, boxes_m)
-        msm = PD.max_over_ranks([timed_device_steps(step_mapper, K, W, barrier)], dev)[0]
+        msm = PD.max_over_ranks([timed_device_steps(step_mapper, K, W, barrier)[0]], dev)[0]
         mflow = {"value": K * B * world * 100.0 / (msm / 1e3), "unit": "masks/s", "ms_per_step": msm / K,
                  "fused_task_heads": bool(fused_m), "geometry": "1024x768 valid region of the padded 1024^2 input -> 480x640 outputs"}
 
@@ -566,7 +609,11 @@ def main():
     ap.add_argument("--acc-images", type=int, default=0,
                     help="held images per rank scored against the oracle (0 = 16 images divided over the ranks, at least 2)")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
         run_reference(args, rank, world)
