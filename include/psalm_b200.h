@@ -292,6 +292,35 @@ int psalm_patch_merge_layernorm(const void* x, const void* weight, const void* b
 int psalm_region_pool(const void* tokens, const float* points, const int* region_image, void* out, int B, int h, int w,
                       int C, int R, int P, int dtype, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * COCO run-length encoding of binary masks (csrc/rle.cu), byte for byte what pycocotools' maskApi.c rleEncode +
+ * rleToString produce.  Replaces `pycocotools.mask.encode` as called on the dense masks of eval_seg's results, after
+ * a copy of the dense masks to the host: detectron2's instances_to_coco_json behind COCOEvaluator.process
+ * (psalm/eval/instance_segmentation.py:128,150; instance_evaluation.py:13,17) and the region script
+ * (psalm/eval/region_segmentation.py:282-283).
+ *   masks   [K,H,W] contiguous, row-major, dtype PSALM_F32 / F16 / BF16 / U8 (uint8 or bool).  A pixel is foreground
+ *           when its value is non-zero; masks are expected to hold 0 / 1 (other values, NaN included, are outside the
+ *           contract).  K >= 1, H, W >= 1, H * W < 2^31.
+ *   counts  uint32 run lengths of every mask in COLUMN-MAJOR pixel order, alternating 0-runs and 1-runs and starting
+ *           with a 0-run (of length 0 when pixel (0, 0) is set); mask k's runs are counts[run_offsets[k] ..
+ *           run_offsets[k+1]).
+ *   strings the compressed counts strings of rleToString, mask k's at strings[str_offsets[k] .. str_offsets[k+1])
+ *           (no terminating NUL).
+ * Three calls on one stream, each sizing the output of the next, so that every buffer has its exact size:
+ *   psalm_mask_rle_sizes   -> run_offsets [K+1] int64 (read run_offsets[K] to size `counts`)
+ *   psalm_mask_rle_runs    -> counts, str_offsets [K+1] int64 (read str_offsets[K] to size `strings`)
+ *   psalm_mask_rle_write   -> strings
+ * `workspace` (psalm_mask_rle_workspace_bytes(K, H, W) bytes: the masks as column-major bits + 8 bytes per column) is
+ * written by _sizes and read by _runs.
+ * ------------------------------------------------------------------------------------------ */
+size_t psalm_mask_rle_workspace_bytes(int K, int H, int W);
+int psalm_mask_rle_sizes(const void* masks, void* workspace, size_t workspace_bytes, int64_t* run_offsets, int K, int H,
+                         int W, int dtype, void* stream);
+int psalm_mask_rle_runs(const void* workspace, size_t workspace_bytes, const int64_t* run_offsets, uint32_t* counts,
+                        int64_t* str_offsets, int K, int H, int W, void* stream);
+int psalm_mask_rle_write(const uint32_t* counts, const int64_t* run_offsets, const int64_t* str_offsets, char* strings,
+                         int K, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -65,6 +65,10 @@ SIGNATURES = {
     "psalm_linear_fused": ([_c_vp, ctypes.c_longlong, _c_vp, _c_vp, _c_vp, ctypes.c_longlong, _c_i, _c_i, _c_i,
                             ctypes.c_longlong, _c_i, _c_vp], _c_i),
     "psalm_groupnorm_tokens": ([_c_vp] * 6 + [_c_i] * 4 + [ctypes.c_float, _c_i, _c_i, _c_vp], _c_i),
+    "psalm_mask_rle_workspace_bytes": ([_c_i] * 3, ctypes.c_size_t),
+    "psalm_mask_rle_sizes": ([_c_vp, _c_vp, ctypes.c_size_t, _c_vp] + [_c_i] * 4 + [_c_vp], _c_i),
+    "psalm_mask_rle_runs": ([_c_vp, ctypes.c_size_t, _c_vp, _c_vp, _c_vp] + [_c_i] * 3 + [_c_vp], _c_i),
+    "psalm_mask_rle_write": ([_c_vp] * 4 + [_c_i, _c_vp], _c_i),
 }
 
 

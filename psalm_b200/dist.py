@@ -69,8 +69,9 @@ def pack_predictions(results, num_queries=100):
 def pack_mask_bits(masks):
     """Instance masks [n, H, W] (float 0/1 or bool, as `Instances.pred_masks`) -> bit-packed uint8 [n, H, ceil(W/8)]
     (MSB = leftmost pixel, numpy.packbits order): 1/32 of the bytes of the dense float masks of the reference API, the
-    form in which they cross NVLink / PCIe to the evaluators (RLE encoding stays on the host, pycocotools).  Torch ops
-    only: runs on the device that holds the masks."""
+    form in which they cross NVLink / PCIe between ranks.  COCO evaluators take the RLE encoded on the device instead
+    (`psalm_b200.coco.encode` / `instances_to_coco_json`, a few kilobytes per mask).  Torch ops only: runs on the device
+    that holds the masks."""
     n, H, W = masks.shape
     b = masks > 0 if masks.dtype != torch.bool else masks
     pad = (-W) % 8

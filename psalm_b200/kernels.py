@@ -350,6 +350,49 @@ def region_pool(tokens, points, region_image, h, w):
     return out
 
 
+_RLE_DT = {torch.float32: _lib.F32, torch.float16: _lib.F16, torch.bfloat16: _lib.BF16, torch.uint8: _lib.U8,
+           torch.bool: _lib.U8}
+
+
+@_on_device
+def mask_rle(masks):
+    """Binary masks [K,H,W] (K >= 1; fp32 / fp16 / bf16 / uint8 / bool, non-zero = foreground) -> the COCO RLE of every mask
+    (pycocotools maskApi.c rleEncode + rleToString, csrc/rle.cu) on the current stream:
+      counts      uint32 [sum of run counts] run lengths in column-major order, mask k's at run_offsets[k]:run_offsets[k+1]
+      run_offsets int64 [K+1] on the device
+      strings     uint8 [sum of string lengths] the compressed counts strings, on the device
+      str_offsets int64 [K+1] on the host: mask k's string is strings[str_offsets[k]:str_offsets[k+1]].
+    Two small host synchronisations (the total run count, then the string offsets) size the outputs exactly."""
+    _chk(masks, "mask_rle.masks")
+    if masks.dim() != 3 or masks.shape[0] == 0:
+        raise _lib.PsalmKernelError("mask_rle: expected masks [K,H,W] with K >= 1, got %s" % (tuple(masks.shape),))
+    if masks.dtype not in _RLE_DT:
+        raise _lib.PsalmKernelError("mask_rle: unsupported dtype %s" % masks.dtype)
+    K, H, W = masks.shape
+    dev = masks.device
+    L = _lib.lib()
+    st = _lib.stream_ptr(dev)
+    ws = torch.empty(L.psalm_mask_rle_workspace_bytes(K, H, W), dtype=torch.uint8, device=dev)
+    run_offsets = torch.empty(K + 1, dtype=torch.int64, device=dev)
+    rc = L.psalm_mask_rle_sizes(_lib.ptr(masks), _lib.ptr(ws), ws.numel(), _lib.ptr(run_offsets), K, H, W,
+                                _RLE_DT[masks.dtype], st)
+    _lib.check(rc, "psalm_mask_rle_sizes")
+    _count(4)
+    counts = torch.empty(int(run_offsets[K].item()), dtype=torch.int32, device=dev).view(torch.uint32)   # host sync 1
+    str_offsets_dev = torch.empty(K + 1, dtype=torch.int64, device=dev)
+    rc = L.psalm_mask_rle_runs(_lib.ptr(ws), ws.numel(), _lib.ptr(run_offsets), _lib.ptr(counts),
+                               _lib.ptr(str_offsets_dev), K, H, W, st)
+    _lib.check(rc, "psalm_mask_rle_runs")
+    _count(3)
+    str_offsets = str_offsets_dev.cpu()                                                                      # host sync 2
+    strings = torch.empty(int(str_offsets[K]), dtype=torch.uint8, device=dev)
+    rc = L.psalm_mask_rle_write(_lib.ptr(counts), _lib.ptr(run_offsets), _lib.ptr(str_offsets_dev),
+                                _lib.ptr(strings), K, st)
+    _lib.check(rc, "psalm_mask_rle_write")
+    _count()
+    return counts, run_offsets, strings, str_offsets
+
+
 LINEAR_FUSED = True   # False: library GEMM + separate elementwise pass (A/B runs)
 _EPILOGUES = {"bias": 0, "gelu_erf": 1, "head_major": 2}
 
